@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- haystack GB/s scanned (+ matches/s) for find_matches_as_indexes on the BASELINE.json workloads.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 2|3|4|5]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config 2|3|4|5] [--dump-outputs DIR]
 
 --config (default 2, the configuration BASELINE.json's metric is quoted on at one GPU):
   2  benchmarks/names.txt patterns (4 244), Implementation.DFA, 100k x 4 KiB synthetic UTF-8 haystacks, AhoCorasick
@@ -16,6 +16,10 @@ public host-buffer API (scan_host: pinned host memory in, host arrays out, H2D/D
 timed region the result of one batch is compared with the CPU oracle ("verified").  `--impl reference` times the
 reference's CPU path: the Rust crate cannot be built in this image, so that arm runs the C oracle port (oracle/) on all
 host cores and says so in cpu_baseline.kind = "port".
+
+`--dump-outputs DIR` writes what the last timed step returned (rank 0's match list, match offsets and total; with several
+GPUs also the gathered list) as DIR/<name>.npy in float64.  The inputs are seeded, so two builds run with the same
+arguments can be compared file for file.
 """
 from __future__ import annotations
 
@@ -243,6 +247,33 @@ def emit(line):
     out.flush()
 
 
+DUMP_BYTES = 64_000_000   # --dump-outputs writes at most this much, .npy headers included
+
+
+def write_outputs(out_dir, arrays, limit=DUMP_BYTES, seed=0):
+    """--dump-outputs: each array as out_dir/<name>.npy in float64 (the values are integers below 2^53, so exact).
+    Smallest first, each array gets an equal share of the `limit` bytes not yet written; one larger than its share
+    keeps a sample of its rows, drawn with a fixed seed and kept in order, and out_dir/<name>_rows.npy holds the
+    numbers of the rows kept.  Two builds that computed the same lists write the same files."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: np.asarray(v) for k, v in arrays.items()}
+    room = limit - 512 * len(arrays)   # (.npy headers)
+    for i, name in enumerate(sorted(arrays, key=lambda k: (arrays[k].size, k))):
+        a = arrays[name]
+        share = room // (len(arrays) - i)
+        rows_path = os.path.join(out_dir, name + "_rows.npy")
+        if a.size * 8 > share and a.ndim:
+            keep = share // (8 * (a.size // a.shape[0] + 1))   # a kept row costs its values and its row number
+            rows = np.sort(np.random.default_rng(seed).choice(a.shape[0], size=keep, replace=False))
+            a = a[rows]
+            np.save(rows_path, rows.astype(np.float64))
+            room -= 8 * keep
+        elif os.path.exists(rows_path):
+            os.remove(rows_path)   # left by an earlier, sampled dump into the same directory
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
+        room -= 8 * a.size
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -260,7 +291,14 @@ def main():
     ap.add_argument("--kernel", type=int, default=0, help=argparse.SUPPRESS)
     ap.add_argument("--hot-rows", type=int, default=0, help=argparse.SUPPRESS)
     ap.add_argument("--table", type=int, default=0, help=argparse.SUPPRESS)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results (match list, per-haystack match "
+                                                           "offsets, total; on rank 0, and the gathered list with several GPUs) "
+                                                           "as DIR/<name>.npy in float64, at most 64 MB in all (a seeded sample of rows beyond that)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm counts matches, it keeps no match list")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     claim_stdout()
 
@@ -391,6 +429,23 @@ def main():
     ev1.record()
     host_enqueue_ms = (time.perf_counter() - host_t0) * 1e3 / max(args.steps, 1)
     torch.cuda.synchronize()
+    if args.dump_outputs and rank == 0:
+        # now, before a later scan reuses the last step's workspace slot
+        if big:
+            matches, total = out, tot
+        else:
+            status = tot.tolist()   # sync=False: the device status, read as scan_device reads it when it synchronises
+            total = status[0]
+            assert status[1] or total == status[4] == 0, "the last timed step's match list did not fit its capacity"
+            matches = out[:total]
+        dump = {"matches": matches, "match_offsets": moffs, "total": np.array(total)}
+        if world > 1:
+            dump["gathered_matches"] = decode_gathered(gathered) if gather is not None else gathered
+        for k, v in dump.items():
+            if isinstance(v, torch.Tensor):
+                v = v.cpu().numpy()
+                dump[k] = v.view(np.uint32) if v.dtype == np.int32 else v
+        write_outputs(args.dump_outputs, dump)
     if world > 1:
         dist.barrier()
     clocks = sampler.stop()
