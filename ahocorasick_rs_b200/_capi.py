@@ -12,6 +12,7 @@ LIB_PATH = os.environ.get("ACB200_LIB") or os.path.join(HERE, "libacb200.so")
 
 ACB_OK = 0
 ACB_EINVAL, ACB_EBUILD, ACB_EUNSUPPORTED, ACB_ECUDA, ACB_ECAPACITY = -1, -2, -3, -4, -5
+ACB_ASCII_CASE_INSENSITIVE = 1   # acb_build_ex flag
 
 
 class Plan(C.Structure):
@@ -63,6 +64,9 @@ def lib():
         L.acb_timing_enable.argtypes = [C.c_int]
         L.acb_timing_read.argtypes = [C.POINTER(C.c_double), C.POINTER(C.c_uint64)]
         L.acb_build.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.c_int, C.POINTER(C.c_void_p)]
+        L.acb_build_ex.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_int, C.c_int, C.c_uint32, C.POINTER(C.c_void_p)]
+        L.acb_build_flags.restype = C.c_uint32
+        L.acb_build_flags.argtypes = [C.c_void_p]
         L.acb_free.argtypes = [C.c_void_p]
         for name, res in [("acb_num_patterns", C.c_uint64), ("acb_num_states", C.c_uint64),
                           ("acb_num_columns", C.c_uint32), ("acb_max_pattern_len", C.c_uint32),
@@ -120,4 +124,5 @@ EXPORTS = [
     "acb_launch_count", "acb_set_tuning", "acb_timing_enable", "acb_timing_read",
     "acb_profile", "acb_hot_bytes", "acb_hot_build", "acb_hot_rows", "acb_hot_describe",
     "acb_sieve_build", "acb_sieve_write", "acb_sieve_describe", "acb_pack_gather_block", "acb_select_non_overlapping",
+    "acb_build_ex", "acb_build_flags",
 ]

@@ -15,6 +15,8 @@
 #include <stdexcept>
 #include <thread>
 
+#include "sieve.h"  // ascii_fold: the one fold the builders and the sieve kernel share
+
 namespace acb {
 namespace {
 
@@ -56,11 +58,14 @@ inline uint64_t align16(uint64_t x) { return (x + 15) & ~uint64_t(15); }
 }  // namespace
 
 Automaton *build_automaton(const uint8_t *blob, const uint64_t *offsets, uint64_t n, int match_kind,
-                           int implementation) {
+                           int implementation, uint32_t flags) {
     if (match_kind < 0 || match_kind > 2) throw std::runtime_error("unknown match kind");
     if (n >= 0x7fffffffull) throw std::runtime_error("too many patterns: pattern ids must fit in 31 bits");
     const bool leftmost = match_kind != 0;
     const bool leftmost_first = match_kind == 1;
+    // case-insensitive: the trie holds the folded patterns and the column map sends both cases of a letter to one
+    // column, so the scan kernels see folded text without folding anything themselves
+    const bool fold = (flags & kAsciiCaseInsensitive) != 0;
 
     // ---- 1. trie -----------------------------------------------------------
     TrieBuilder tb;
@@ -88,9 +93,10 @@ Automaton *build_automaton(const uint8_t *blob, const uint64_t *offsets, uint64_
                 shadowed = true;
                 break;
             }
-            used[p[k]] = true;
-            uint32_t c = tb.child(s, p[k]);
-            if (c == TrieBuilder::kNone) c = tb.add_child(s, p[k]);
+            const uint8_t b = fold ? static_cast<uint8_t>(ascii_fold(p[k])) : p[k];
+            used[b] = true;
+            uint32_t c = tb.child(s, b);
+            if (c == TrieBuilder::kNone) c = tb.add_child(s, b);
             s = c;
         }
         if (shadowed) continue;
@@ -211,9 +217,13 @@ Automaton *build_automaton(const uint8_t *blob, const uint64_t *offsets, uint64_
     if (n_used == 0) lo = hi = 0;
     const uint32_t class_cols = n_used + 1;    // column 0 = every byte no pattern uses
     const uint32_t range_cols = hi - lo + 2;   // last column = every byte outside [lo, hi]
+    // kColRange computes the column arithmetically in the kernels: it cannot send 'A' to the column of 'a', so a
+    // case-insensitive automaton whose patterns hold a letter takes the class map
+    bool letters = false;
+    for (uint32_t b = 'a'; b <= 'z'; b++) letters |= used[b];
     uint32_t col_mode, n_cols;
     uint8_t colmap[256];
-    if (range_cols * 4 <= class_cols * 5 && range_cols <= 256) {
+    if (range_cols * 4 <= class_cols * 5 && range_cols <= 256 && !(fold && letters)) {
         col_mode = kColRange;
         n_cols = range_cols;
         for (uint32_t b = 0; b < 256; b++) colmap[b] = static_cast<uint8_t>(std::min(b - lo, n_cols - 1));  // unsigned wrap for b < lo
@@ -227,6 +237,8 @@ Automaton *build_automaton(const uint8_t *blob, const uint64_t *offsets, uint64_
             uint32_t next = 1;
             for (uint32_t b = 0; b < 256; b++) colmap[b] = used[b] ? static_cast<uint8_t>(next++) : 0;
         }
+        if (fold)
+            for (uint32_t b = 'A'; b <= 'Z'; b++) colmap[b] = colmap[b | 0x20u];
     }
 
     // ---- 5. image ---------------------------------------------------------------
@@ -249,6 +261,7 @@ Automaton *build_automaton(const uint8_t *blob, const uint64_t *offsets, uint64_
     h.max_pat_len = max_len;
     h.min_pat_len = min_len;
     h.n_hot_eligible = n_states;
+    h.flags = flags & kAsciiCaseInsensitive;
     uint64_t off = align16(sizeof(ImageHeader));
     h.off_colmap = off;
     off = align16(off + 256);

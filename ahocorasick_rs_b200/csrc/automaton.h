@@ -35,7 +35,7 @@ struct ImageHeader {
     uint32_t max_pat_len;
     uint32_t min_pat_len;
     uint32_t n_hot_eligible; // states are BFS ordered; rows [0, n_hot_eligible) may be cached on chip
-    uint32_t reserved;
+    uint32_t flags;          // kAsciiCaseInsensitive (sieve.h): the trie holds the folded patterns, colmap folds the text
     uint64_t off_colmap;     // u8[256]
     uint64_t off_trans;      // u32[n_states * n_cols]: next state | kMatchFlag
     uint64_t off_match_off;  // u32[n_states + 1]
@@ -85,9 +85,9 @@ struct Automaton {
     uint32_t sieve_bloom_max = 0, sieve_w_max = 0;
 };
 
-// Builds the automaton; throws std::runtime_error with a message on failure.
+// Builds the automaton; throws std::runtime_error with a message on failure.  flags: kAsciiCaseInsensitive or 0.
 Automaton *build_automaton(const uint8_t *blob, const uint64_t *offsets, uint64_t n, int match_kind,
-                           int implementation);
+                           int implementation, uint32_t flags);
 
 // Size of / builder for the hot image with at most max_rows rows.  visits may be
 // null (no profile yet: breadth-first prefix) or n_states sampled visit counts.

@@ -709,18 +709,26 @@ int acb_set_tuning(const acb_tuning *t) {
     return ACB_OK;
 }
 
-int acb_build(const uint8_t *blob, const uint64_t *offsets, uint64_t n, int match_kind, int implementation,
-              acb_automaton **out) {
+int acb_build_ex(const uint8_t *blob, const uint64_t *offsets, uint64_t n, int match_kind, int implementation, uint32_t flags,
+                 acb_automaton **out) {
     if (!out || !offsets || (!blob && n && offsets[n] != 0)) return fail(ACB_EINVAL, "null argument");
     if (implementation < -1 || implementation > 2) return fail(ACB_EINVAL, "unknown implementation");
+    if (flags & ~uint32_t(ACB_ASCII_CASE_INSENSITIVE)) return fail(ACB_EINVAL, "unknown build flags");
     try {
-        Automaton *impl = build_automaton(blob, offsets, n, match_kind, implementation);
+        Automaton *impl = build_automaton(blob, offsets, n, match_kind, implementation, flags);
         *out = new acb_automaton{impl};
         return ACB_OK;
     } catch (const std::exception &e) {
         return fail(ACB_EBUILD, e.what());
     }
 }
+
+int acb_build(const uint8_t *blob, const uint64_t *offsets, uint64_t n, int match_kind, int implementation,
+              acb_automaton **out) {
+    return acb_build_ex(blob, offsets, n, match_kind, implementation, 0u, out);
+}
+
+uint32_t acb_build_flags(const acb_automaton *a) { return a->impl->hdr.flags; }
 
 void acb_free(acb_automaton *a) {
     if (!a) return;
@@ -776,7 +784,7 @@ uint64_t acb_sieve_build(acb_automaton *a, uint32_t bloom_bytes_max, uint32_t w_
     std::lock_guard<std::mutex> lock(A.sieve_mutex);
     if (A.sieve.empty() || A.sieve_bloom_max != bloom_bytes_max || A.sieve_w_max != w_max) {
         try {
-            sieve_image_build(A.pat_blob.data(), A.pat_offs.data(), A.hdr.n_patterns, bloom_bytes_max, w_max, A.sieve);
+            sieve_image_build(A.pat_blob.data(), A.pat_offs.data(), A.hdr.n_patterns, bloom_bytes_max, w_max, A.hdr.flags, A.sieve);
             A.sieve_bloom_max = bloom_bytes_max;
             A.sieve_w_max = w_max;
         } catch (const std::exception &e) {
@@ -1051,7 +1059,7 @@ DevSieve make_sieve_view(const SieveHeader &h, const void *dev_sieve) {
 }
 
 template <bool CP>
-int launch_sieve(const DevSieve &sv, const Batch &B, SievePlan &P, const Sink &out, uint32_t *task_cont, uint32_t *hay_cont,
+int launch_sieve(const DevSieve &sv, bool fold, const Batch &B, SievePlan &P, const Sink &out, uint32_t *task_cont, uint32_t *hay_cont,
                  unsigned int *task_counter, const DeviceInfo &d, cudaStream_t st) {
     // as many windows of text per warp as fit next to the filters (a power of two): the more, the fuller the rounds of
     // the later stages when survivors are rare
@@ -1061,9 +1069,10 @@ int launch_sieve(const DevSieve &sv, const Batch &B, SievePlan &P, const Sink &o
     const uint32_t smem = sieve_smem_bytes(filter_bytes, ring, CP);
     if (smem > (uint32_t)d.max_smem_optin) return fail(ACB_ECUDA, "the sieve's filters do not fit in shared memory (rebuild them with a smaller bloom_bytes_max)");
     P.ring = ring;
+    // (a case-insensitive image: the kernel variant that folds the text as it loads it)
 #define ACB_SIEVE_GO(WC)                                                                                  \
     do {                                                                                                  \
-        auto kern = sieve_scan_kernel<CP, WC>;                                                            \
+        auto kern = fold ? sieve_scan_kernel<CP, WC, true> : sieve_scan_kernel<CP, WC, false>;            \
         CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, d.max_smem_optin)); \
         kern<<<d.sms, kSieveThreads, smem, st>>>(sv, B, P, out, task_cont, hay_cont, task_counter);       \
     } while (0)
@@ -1256,8 +1265,9 @@ int acb_scan_batch(const acb_automaton *a, const void *dev_image, const void *de
         // code points: the continuation bytes each task saw before a haystack that starts in it, per haystack; lives in
         // the match_offsets buffer until the epilogue's last phases write the offsets there
         uint32_t *hay_cont = reinterpret_cast<uint32_t *>(match_offsets);
-        rc = cp ? launch_sieve<true>(sv, B, SP, out, cont_tail, hay_cont, task_counter, d, st)
-                : launch_sieve<false>(sv, B, SP, out, cont_tail, hay_cont, task_counter, d, st);
+        const bool fold = (sh.flags & kAsciiCaseInsensitive) != 0;
+        rc = cp ? launch_sieve<true>(sv, fold, B, SP, out, cont_tail, hay_cont, task_counter, d, st)
+                : launch_sieve<false>(sv, fold, B, SP, out, cont_tail, hay_cont, task_counter, d, st);
         if (rc) return rc;
         CUDA_OK(cudaGetLastError());
         if (e1) {

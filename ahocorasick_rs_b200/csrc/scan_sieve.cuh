@@ -129,9 +129,13 @@ __device__ __forceinline__ uint32_t warp_excl_scan(uint32_t v, uint32_t lane, ui
 }
 
 // WC: 0 = W < 4 (the window word is shifted down), 1 = W == 4, 2 = W in 6..8 (two words), 3 = W == 5 (a word and a byte)
+// FOLD: the image was built case-insensitively (sieve.h, kAsciiCaseInsensitive): text is folded where it enters registers
+// -- the carry before the task's first window and every window as it becomes the current one (ascii_fold4, 4 bytes per
+// instruction group) -- and the one byte per step stage 2 reads from global memory.  Everything else (the fast path, the
+// ring and its history, stage 1, the code point counts) then sees folded bytes; the fold never touches a byte >= 0x80.
 //
 // Positions inside a task are 32-bit offsets from the task's start (`rel`); the 64-bit stream position is t_lo + rel.
-template <bool CP, int WC>
+template <bool CP, int WC, bool FOLD>
 __global__ void __launch_bounds__(kSieveThreads, 1)
 sieve_scan_kernel(DevSieve sv, Batch B, SievePlan P, Sink out, uint32_t *task_cont, uint32_t *hay_cont, unsigned int *task_counter) {
     extern __shared__ __align__(128) uint8_t smem[];
@@ -309,7 +313,8 @@ sieve_scan_kernel(DevSieve sv, Batch B, SievePlan P, Sink out, uint32_t *task_co
                     if (na.y & kNodeTerminal) best = v;
                     const uint32_t nk = (na.y >> 8) & 0x1ffu;
                     if (nk == 0 || (int32_t)rel - (int32_t)d < hs) break;  // no longer pattern, or it would start before the haystack
-                    const uint32_t b = __ldg(tptr + ((int64_t)(int32_t)rel - (int64_t)d));
+                    uint32_t b = __ldg(tptr + ((int64_t)(int32_t)rel - (int64_t)d));
+                    if (FOLD) b = ascii_fold(b);
                     uint32_t c = kSieveNoNode;
                     uint2 nc = make_uint2(0, 0);
                     if (nk <= 8) {
@@ -431,14 +436,20 @@ sieve_scan_kernel(DevSieve sv, Batch B, SievePlan P, Sink out, uint32_t *task_co
             __syncwarp();
         };
 
+        // case-insensitive: the text as the image expects it (the next window is folded when it becomes the current one,
+        // not at its load: the load stays in flight while this window is scanned)
+        auto fold16 = [&](uint4 v) -> uint4 {
+            if (FOLD) v = make_uint4(ascii_fold4(v.x), ascii_fold4(v.y), ascii_fold4(v.z), ascii_fold4(v.w));
+            return v;
+        };
         uint32_t carry_z = 0, carry_w = 0;
         {
-            const uint4 c = load16(wrel - 16);
+            const uint4 c = fold16(load16(wrel - 16));
             carry_z = c.z;
             carry_w = c.w;
             if (lane == 0) sts128(text_s(wrel) - 16, c);
         }
-        uint4 cur = load16(wrel + 16 * lane);
+        uint4 cur = fold16(load16(wrel + 16 * lane));
         uint4 nxt = make_uint4(0, 0, 0, 0);
         uint32_t cur_slot = slot_s(wrel);  // the ring slot of the current window
 
@@ -583,6 +594,7 @@ sieve_scan_kernel(DevSieve sv, Batch B, SievePlan P, Sink out, uint32_t *task_co
             carry_z = __shfl_sync(0xffffffffu, cur.z, 31);
             carry_w = __shfl_sync(0xffffffffu, cur.w, 31);
             cur = nxt;
+            if (FOLD) cur = fold16(cur);
         }
         if (lane == 0) out.unit_counts[task] = n_emitted;
         if (CP && lane == 0) task_cont[task] = cp_before;

@@ -46,7 +46,15 @@ void filter_insert(std::vector<uint32_t> &bits, uint32_t base, uint32_t n_words,
 }  // namespace
 
 uint64_t sieve_image_build(const uint8_t *blob, const uint64_t *offsets, uint64_t n, uint32_t bloom_bytes_max, uint32_t w_max,
-                           std::vector<uint8_t> &out) {
+                           uint32_t flags, std::vector<uint8_t> &out) {
+    // case-insensitive: everything below is built from the folded patterns (the image equals the case-sensitive image
+    // of the folded pattern list but for the flag)
+    std::vector<uint8_t> folded;
+    if (flags & kAsciiCaseInsensitive) {
+        folded.assign(blob, blob + (n ? offsets[n] : 0));
+        for (auto &b : folded) b = (uint8_t)ascii_fold(b);
+        blob = folded.data();
+    }
     uint32_t min_len = 0xffffffffu, max_len = 0;
     bool used[256] = {false};
     for (uint64_t i = 0; i < n; i++) {
@@ -286,6 +294,7 @@ uint64_t sieve_image_build(const uint8_t *blob, const uint64_t *offsets, uint64_
     h.n_keys = n_keys;
     h.n_filter_entries = (uint32_t)std::min<uint64_t>(entries, 0xffffffffull);
     h.prim_words = prim_words;
+    h.flags = flags & kAsciiCaseInsensitive;
     for (uint32_t d = 1; d <= kSieveMaxLevel; d++)
         if (d <= level_cap && terms_at[d]) h.term_levels |= 1u << d;
     uint64_t off = align16(sizeof(SieveHeader));

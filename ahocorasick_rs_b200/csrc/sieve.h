@@ -79,6 +79,20 @@ ACB_HD uint32_t sieve_mulhi(uint32_t a, uint32_t b) { return (uint32_t)(((uint64
 ACB_HD uint32_t sieve_probe_word(uint32_t p, uint32_t n_words) { return sieve_mulhi(p, n_words); }
 ACB_HD uint32_t sieve_probe_bit(uint32_t p) { return p & 31u; }
 
+// ---- ASCII case folding ---------------------------------------------------------------------
+// Built with kAsciiCaseInsensitive, the image holds the FOLDED patterns and the scan folds the text before it hashes or
+// compares a byte: an ASCII upper-case letter (0x41-0x5A) becomes its lower-case form (| 0x20), every other byte --
+// bytes >= 0x80 included, so no UTF-8 sequence changes -- stays as it is.
+constexpr uint32_t kAsciiCaseInsensitive = 1u;  // = ACB_ASCII_CASE_INSENSITIVE (include/acb200.h)
+ACB_HD uint32_t ascii_fold(uint32_t b) { return b - 0x41u < 26u ? (b | 0x20u) : b; }
+// the same for the four bytes of a word: a byte is upper case when its top bit is clear and its low seven bits are
+// >= 0x41 (t + 0x3f carries into bit 7) and not >= 0x5b (t + 0x25 does not); no sum carries into the next byte
+ACB_HD uint32_t ascii_fold4(uint32_t w) {
+    const uint32_t t = w & 0x7f7f7f7fu;
+    const uint32_t upper = (t + 0x3f3f3f3fu) & ~(t + 0x25252525u) & ~w & 0x80808080u;
+    return w | (upper >> 2);
+}
+
 // ---- the image ------------------------------------------------------------------------------
 // All offsets are bytes from the start of the image, 16-byte aligned.
 struct SieveHeader {
@@ -96,7 +110,8 @@ struct SieveHeader {
     uint32_t n_filter_entries;
     uint32_t prim_words;   // the primary bitmap: ONE bit per W-byte suffix, kept sparse (the fast path tests only this)
     uint32_t term_levels;  // bit d: some pattern is exactly d bytes long (d <= 16): only those levels carry end marks
-    uint32_t pad1, pad2;
+    uint32_t flags;        // kAsciiCaseInsensitive: built from the folded patterns, the scan folds the text
+    uint32_t pad2;
     uint64_t off_bloom;    // u32[bloom_words]
     uint64_t off_ht;       // SieveSlot[ht_mask + 1]
     uint64_t off_node_a;   // SieveNodeA[n_nodes]
@@ -131,8 +146,8 @@ constexpr uint32_t kNodeTerminal = 1u << 17;
 struct Automaton;
 // Builds the sieve image for the automaton's patterns.  bloom_bytes_max: the shared memory the filters may take when the
 // scan keeps one window of text per warp on chip (the builder may use less, to leave room for a deeper ring: sieve.cpp).
-// w_max: cap on the primary window (0 = automatic).
+// w_max: cap on the primary window (0 = automatic).  flags: kAsciiCaseInsensitive or 0.
 uint64_t sieve_image_build(const uint8_t *blob, const uint64_t *offsets, uint64_t n, uint32_t bloom_bytes_max, uint32_t w_max,
-                           std::vector<uint8_t> &out);
+                           uint32_t flags, std::vector<uint8_t> &out);
 
 }  // namespace acb

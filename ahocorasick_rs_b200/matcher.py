@@ -114,7 +114,8 @@ class _Automaton:
     """Owns the host automaton handle, its device image and a growable device
     workspace.  Shared by both public classes."""
 
-    def __init__(self, pattern_bytes: Sequence[bytes], matchkind: MatchKind, implementation: Optional[Implementation]):
+    def __init__(self, pattern_bytes: Sequence[bytes], matchkind: MatchKind, implementation: Optional[Implementation],
+                 ascii_case_insensitive: bool = False):
         L = _capi.lib()
         n = len(pattern_bytes)
         offs = np.zeros(n + 1, dtype=np.uint64)
@@ -123,13 +124,15 @@ class _Automaton:
         blob = np.frombuffer(b"".join(pattern_bytes) or b"\0", dtype=np.uint8)
         h = C.c_void_p()
         impl = -1 if implementation is None else implementation.value
-        rc = L.acb_build(blob.ctypes.data, offs.ctypes.data, n, matchkind.value, impl, C.byref(h))
+        flags = _capi.ACB_ASCII_CASE_INSENSITIVE if ascii_case_insensitive else 0
+        rc = L.acb_build_ex(blob.ctypes.data, offs.ctypes.data, n, matchkind.value, impl, flags, C.byref(h))
         if rc != _capi.ACB_OK:
             raise ValueError(_capi.last_error())
         self._h = h
         self._L = L
         self.matchkind = matchkind
         self.implementation = implementation
+        self.ascii_case_insensitive = bool(ascii_case_insensitive)
         self.n_patterns = n
         self.num_states = int(L.acb_num_states(h))
         self.num_columns = int(L.acb_num_columns(h))
@@ -727,6 +730,11 @@ def _as_buffer_bytes(obj) -> bytes:
     return obj if isinstance(obj, bytes) else (mv if mv.format == "B" else mv.cast("B"))
 
 
+def _check_ascii_case_insensitive(value):
+    if not isinstance(value, bool):
+        raise TypeError("ascii_case_insensitive must be a bool")
+
+
 def _tuples(m: np.ndarray):
     return list(zip(m[:, 1].tolist(), m[:, 2].tolist(), m[:, 3].tolist()))
 
@@ -740,14 +748,19 @@ class AhoCorasick:
     * ``store_patterns``: keep references to the patterns to speed up
       ``find_matches_as_strings``; ``None`` = store iff total length <= 4096 code points.
     * ``implementation``: ``Implementation`` hint or ``None``.
+    * ``ascii_case_insensitive`` (keyword only): an ASCII letter in a pattern matches either case of that letter in
+      the haystack (the crate's ``AhoCorasickBuilder::ascii_case_insensitive``); every other character must match
+      exactly, so ``"é"`` does not match ``"É"``.  Indexes stay code point indexes of the haystack as given.
     """
 
     def __init__(self, patterns: Iterable[str], matchkind: MatchKind = MatchKind.Standard,
-                 store_patterns: Optional[bool] = None, implementation: Optional[Implementation] = None):
+                 store_patterns: Optional[bool] = None, implementation: Optional[Implementation] = None, *,
+                 ascii_case_insensitive: bool = False):
         if not isinstance(matchkind, MatchKind):
             raise TypeError("matchkind must be a MatchKind")
         if implementation is not None and not isinstance(implementation, Implementation):
             raise TypeError("implementation must be an Implementation or None")
+        _check_ascii_case_insensitive(ascii_case_insensitive)
         it = iter(patterns)  # TypeError for non-iterables, like try_iter()? at src/lib.rs:147
         strs = []
         encoded = []
@@ -772,7 +785,7 @@ class AhoCorasick:
                 strs.append(p)
             encoded.append(b)
         self._patterns = strs if store else None
-        self._ac = _Automaton(encoded, matchkind, implementation)
+        self._ac = _Automaton(encoded, matchkind, implementation, ascii_case_insensitive)
 
     def find_matches_as_indexes(self, haystack: str, overlapping: bool = False):
         """-> list of (pattern index, start, end) in code points (src/lib.rs:229-249)."""
@@ -783,12 +796,15 @@ class AhoCorasick:
         return _tuples(m)
 
     def find_matches_as_strings(self, haystack: str, overlapping: bool = False):
-        """-> list of matched patterns (src/lib.rs:253-272)."""
+        """-> list of matched patterns (src/lib.rs:253-272).
+
+        With ``ascii_case_insensitive`` the list holds the matched text OF THE HAYSTACK (``"Hello"`` for the pattern
+        ``"hello"``), never the stored pattern, whatever ``store_patterns`` says."""
         if not isinstance(haystack, str):
             raise TypeError("argument 'haystack': 'str' expected")
         self._ac.check_overlapping(overlapping)
         m, _ = self._ac.scan_host_batch([haystack.encode("utf-8")], overlapping, codepoints=True)
-        if self._patterns is not None:
+        if self._patterns is not None and not self._ac.ascii_case_insensitive:
             pats = self._patterns
             return [pats[i] for i in m[:, 1].tolist()]
         return [haystack[s:e] for s, e in zip(m[:, 2].tolist(), m[:, 3].tolist())]
@@ -814,21 +830,25 @@ class AhoCorasick:
 
 class BytesAhoCorasick:
     """Search for multiple pattern bytes against a bytes-like haystack
-    (reference: src/lib.rs:342-363, 366-435).  No references to the patterns are kept."""
+    (reference: src/lib.rs:342-363, 366-435).  No references to the patterns are kept.
+
+    ``ascii_case_insensitive`` (keyword only): an ASCII letter in a pattern matches either case of that letter in the
+    haystack; every other byte, 0x80-0xff included, must match exactly."""
 
     def __init__(self, patterns: Iterable, matchkind: MatchKind = MatchKind.Standard,
-                 implementation: Optional[Implementation] = None):
+                 implementation: Optional[Implementation] = None, *, ascii_case_insensitive: bool = False):
         if not isinstance(matchkind, MatchKind):
             raise TypeError("matchkind must be a MatchKind")
         if implementation is not None and not isinstance(implementation, Implementation):
             raise TypeError("implementation must be an Implementation or None")
+        _check_ascii_case_insensitive(ascii_case_insensitive)
         encoded = []
         for p in iter(patterns):
             b = _as_buffer_bytes(p)
             if len(b) == 0:
                 raise ValueError("You passed in an empty pattern")
             encoded.append(b)
-        self._ac = _Automaton(encoded, matchkind, implementation)
+        self._ac = _Automaton(encoded, matchkind, implementation, ascii_case_insensitive)
 
     def find_matches_as_indexes(self, haystack, overlapping: bool = False):
         """-> list of (pattern index, start, end) in byte offsets (src/lib.rs:422-434)."""

@@ -128,6 +128,24 @@ def config5(n_patterns=50_000, n_haystacks=16_777_216, hay_bytes=4096, seed=5, s
     return pats, data, offs
 
 
+def recase(data, frac=0.5, seed=0):
+    """A copy of `data` (uint8) in which a seeded fraction `frac` of the ASCII letters has the other case: the input
+    of the case-insensitive tests and timings (the matches of a case-insensitive automaton do not change).  Works in
+    slices of 64 MiB so that a full-size batch needs no more than twice its own size."""
+    data = np.asarray(data, dtype=np.uint8)
+    out = np.empty_like(data)
+    rng = np.random.default_rng(seed)
+    flat_in, flat_out = data.reshape(-1), out.reshape(-1)
+    thresh = int(round(frac * 65536))
+    step = 64 << 20
+    for a in range(0, flat_in.size, step):
+        x = flat_in[a:a + step]
+        letter = ((x | np.uint8(0x20)) - np.uint8(0x61)) < 26   # uint8 arithmetic: bytes below 'a' wrap above 26
+        flip = letter & (rng.integers(0, 65536, size=x.size, dtype=np.uint16) < thresh)
+        flat_out[a:a + step] = x ^ (flip.astype(np.uint8) << np.uint8(5))
+    return out
+
+
 def ragged(n_haystacks=1000, max_len=700, alphabet=b"abc", seed=7, empty_frac=0.05):
     """Ragged batch with empty haystacks, for edge-case parity."""
     rng = np.random.default_rng(seed)

@@ -74,6 +74,22 @@ const char *acb_version(void);
  */
 int acb_build(const uint8_t *blob, const uint64_t *offsets, uint64_t n_patterns, int match_kind,
               int implementation, acb_automaton **out);
+
+/*
+ * Build flags (acb_build_ex).
+ * ACB_ASCII_CASE_INSENSITIVE stands in for AhoCorasickBuilder::ascii_case_insensitive(true): an ASCII letter in a
+ * pattern matches either case of that letter in the haystack; no other byte changes (bytes >= 0x80 included, so
+ * code point indexes are unaffected).  The matches are exactly those of the case-sensitive automaton of the folded
+ * patterns (A-Z -> a-z) on the folded haystack, reported with the ORIGINAL pattern ids and lengths; patterns that
+ * differ only in case keep their own ids.
+ */
+#define ACB_ASCII_CASE_INSENSITIVE 1u
+
+/* acb_build with build flags; acb_build(...) == acb_build_ex(..., 0, ...).  Unknown flag bits: ACB_EINVAL. */
+int acb_build_ex(const uint8_t *blob, const uint64_t *offsets, uint64_t n_patterns, int match_kind,
+                 int implementation, uint32_t flags, acb_automaton **out);
+/* The flags the automaton was built with. */
+uint32_t acb_build_flags(const acb_automaton *a);
 void acb_free(acb_automaton *a);
 
 /* Facts about a built automaton. */
